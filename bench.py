@@ -17,6 +17,9 @@ job with all state resident in HBM; e2e = same metric through the C ABI with the
 back every step; roofline = update kernel algorithmic bytes (72 B/particle-step) / its CUDA-event
 duration vs the measured HBM copy peak; cpu_baseline = the CPU oracle (C port, OpenMP) on a bounded
 sample of the same workload.
+
+--dump-outputs DIR writes, after the timed steps, the state the last step left as a caller reads it back (see
+dump_outputs); the inputs depend on the arguments only, so two builds can be compared output for output.
 """
 from __future__ import annotations
 
@@ -51,7 +54,13 @@ def parse_args():
     ap.add_argument("--scaling", default="strong", choices=["strong", "weak"])
     ap.add_argument("--cpu-seconds", type=float, default=12.0, help="budget of the cpu_baseline leg")
     ap.add_argument("--no-cpu-baseline", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the final state of the timed path as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
+    return args
 
 
 # ---------------------------------------------------------------------------------------------------
@@ -231,15 +240,17 @@ class CpuC5:
         return out
 
 
-def measure_cpu_arm(steps: int, warmup: int, budget_s: float):
+def measure_cpu_arm(steps: int, warmup: int, budget_s: float | None):
     """The CPU arm of both the `cpu_baseline` block and `--impl reference`: same workload, same threads, same timing, so
-    that the two agree on the same box. Returns (value over the timed steps, per-step seconds, description dict)."""
+    that the two agree on the same box. `budget_s` lowers `steps` to what fits that many seconds; None times exactly
+    `steps`. Returns (value over the timed steps, per-step seconds, description dict)."""
     n, what = cpu_workload_particles()
     logical, cores, how = usable_cpus()
     arm = CpuC5(n, cores)
     w = arm.timed_steps(max(1, warmup))
     est = min(w)
-    steps = max(1, min(steps, int(budget_s / max(est, 1e-6))))  # exactly the K asked for unless that would take minutes
+    if budget_s is not None:
+        steps = max(1, min(steps, int(budget_s / max(est, 1e-6))))
     ts = arm.timed_steps(steps)
     total = sum(ts)
     med5 = statistics.median((ts + arm.timed_steps(max(0, 5 - steps)))[:5])  # BASELINE.md §3: median of five timed steps
@@ -268,7 +279,7 @@ def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    value, ts, desc, _ = measure_cpu_arm(args.steps, min(args.warmup, 2), 60.0)
+    value, ts, desc, _ = measure_cpu_arm(args.steps, min(args.warmup, 2), None)
     steps = desc["steps"]
     n = desc["particles_per_step"]
     line = {
@@ -288,6 +299,48 @@ def run_reference(args):
 # ---------------------------------------------------------------------------------------------------
 # GPU arm
 # ---------------------------------------------------------------------------------------------------
+DUMP_BLOCK_ROWS = 4096
+DUMP_SAMPLE_ROWS = 128 * DUMP_BLOCK_ROWS  # over the whole job, at 64 B a row (record, indirect row, row number): 32 MiB
+
+
+def dump_sample(rows: int, world: int):
+    """(block, starts): the rows [s, s + block) for s in starts that one of `world` ranks dumps from its `rows`-row shard.
+    The ranks together keep at most DUMP_SAMPLE_ROWS rows; a shard larger than its share is sampled in whole blocks whose
+    positions are drawn from a fixed seed, so the same --particles and --gpus always sample the same rows."""
+    import numpy as np
+    budget = max(1, DUMP_SAMPLE_ROWS // world)
+    if rows <= budget:
+        return rows, np.zeros(1, dtype=np.int64)
+    block = min(DUMP_BLOCK_ROWS, budget)
+    return block, np.sort(np.random.default_rng(0).choice(rows // block, budget // block, replace=False)) * block
+
+
+def dump_outputs(ctx, slab, rows: int, logical_first: int, world: int, out_dir: Path, suffix: str = "") -> None:
+    """Writes what a caller of the simulation reads back after the last step, in the reference layouts:
+      particles.npy  float32 (n, 8)  particle records (position, age, velocity, lifetime)
+      indirect.npy   float64 (n, 3)  {ping, pong, dead} rows of the indirect buffer
+      rows.npy       float64 (n,)    logical row of each of the n sampled rows
+      metadata.npy   float64 (15,)   the effect's metadata row
+      draw_args.npy  float64 (5,)    its draw-indirect args, field by field (base_vertex is signed)
+    float64 holds every u32 and i32 exactly. The rows are those of dump_sample: at most DUMP_SAMPLE_ROWS over the whole job,
+    which keeps all files of all ranks together under 33 MiB. With several GPUs each rank writes the rows of its shard
+    as <name>_rank<r>.npy."""
+    import numpy as np
+    from bevy_hanabi_b200 import recipes
+    block, starts = dump_sample(rows, world)
+    draw = ctx.read_draw_args(0)
+    out = {
+        "particles": np.concatenate([ctx.slab_download_aos(slab, int(s), block, recipes.C5_STRIDE) for s in starts]).view(np.float32),
+        "indirect": np.concatenate([ctx.slab_download_indirect(slab, int(s), block) for s in starts]).astype(np.float64),
+        "rows": (starts[:, None] + np.arange(block) + logical_first).reshape(-1).astype(np.float64),
+        "metadata": np.frombuffer(bytes(ctx.read_metadata(0)), dtype=np.uint32).astype(np.float64),
+        "draw_args": np.array([getattr(draw, f) for f, _ in draw._fields_], dtype=np.float64),
+    }
+    out_dir.mkdir(parents=True, exist_ok=True)
+    for name, a in out.items():
+        np.save(out_dir / f"{name}{suffix}.npy", a)
+
+
 def run_b200(args):
     import torch
     import torch.distributed as dist
@@ -454,6 +507,8 @@ def run_b200(args):
     # hashes its rows under their LOGICAL index; the sum over the shards is independent of how many GPUs hold it)
     mdr = ctx.read_metadata(0)
     assert mdr.alive_count == per_rank and mdr.max_update == per_rank, "bench state corrupted"
+    if args.dump_outputs:
+        dump_outputs(ctx, slab, per_rank, logical_first, n_gpus, Path(args.dump_outputs), f"_rank{rank}" if world > 1 else "")
     frames_run = ctx.frames_simulated
     shard_sum = ctx.slab_checksum(slab, 0, per_rank, index_base=logical_first)
     state_sum = shard_sum

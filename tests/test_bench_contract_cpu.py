@@ -45,3 +45,32 @@ def test_b200_arm_has_no_cpu_path():
     p = subprocess.run([sys.executable, str(ROOT / "bench.py"), "--steps", "2", "--warmup", "3"], capture_output=True, text=True, timeout=300)
     assert p.returncode != 0
     assert "no CUDA device" in (p.stdout + p.stderr) and "{" not in p.stdout
+
+
+@pytest.mark.parametrize("args,message", [(["--steps", "0"], "--steps must be at least 1"),
+                                          (["--impl", "reference", "--dump-outputs", "out"], "--dump-outputs applies to --impl b200")])
+def test_bad_arguments_are_refused(tmp_path, args, message):
+    p = subprocess.run([sys.executable, str(ROOT / "bench.py"), *args], capture_output=True, text=True, timeout=120, cwd=tmp_path)
+    assert p.returncode != 0 and message in p.stderr and "{" not in p.stdout
+    assert not any(tmp_path.iterdir())
+
+
+@pytest.mark.parametrize("particles", [64 << 20, 1 << 20, 1000])
+@pytest.mark.parametrize("world", [1, 2, 3, 8, 200])
+def test_dump_sample_is_capped_over_the_whole_job(world, particles):
+    """--dump-outputs keeps at most DUMP_SAMPLE_ROWS rows over all ranks (64 bytes a row: 32 MiB), the same rows every run."""
+    import numpy as np
+    import bench
+    from bevy_hanabi_b200.sharding import shard_range
+    kept = 0
+    for rank in range(world):
+        first, end = shard_range(particles, rank, world)
+        block, starts = bench.dump_sample(end - first, world)
+        rows = (starts[:, None] + np.arange(block)).reshape(-1)
+        assert np.unique(rows).size == rows.size and 0 <= rows.min() and rows.max() < end - first
+        again = bench.dump_sample(end - first, world)
+        assert again[0] == block and np.array_equal(again[1], starts)
+        kept += rows.size
+    assert kept <= bench.DUMP_SAMPLE_ROWS and kept * 64 <= 32 << 20
+    if particles <= bench.DUMP_SAMPLE_ROWS:
+        assert kept == particles
